@@ -13,8 +13,9 @@ built by ext/__init__.py:18-23; call sites dataset/av_gt_geometry.py:63-78 and m
             grad = sum n_k w_k / sum w_k
 
 Unlike the rest of oracle/, this restatement is PINNED: oracle/Makefile.ref compiles the unmodified reference sources
-into oracle/_ref/nksr_sdfgen_ref.so and tests/test_gpu_sdfgen.py checks both this file and the CUDA kernel against that
-binary on the GPU.  The k-NN search is exact (tinyflann eps = 0, ext/common/kdtree_cuda.cuh:34); scipy's cKDTree stands in.
+into oracle/_ref/nksr_sdfgen_ref.so, tests/golden/sdfgen/sdf_from_points_reference.npz holds that binary's output at a
+sample of the queries, and tests/test_gpu_sdfgen.py checks both this file and the CUDA kernel against it on the GPU.
+The k-NN search is exact (tinyflann eps = 0, ext/common/kdtree_cuda.cuh:34); scipy's cKDTree stands in.
 """
 from __future__ import annotations
 

@@ -1,5 +1,5 @@
 """oracle/sdfgen.py (restatement of ext/sdfgen/sdf_from_points.cu) on the CPU: analytic checks of the rule itself.
-The comparison with the reference BINARY (oracle/_ref) needs a GPU: tests/test_gpu_sdfgen.py."""
+The comparison with the reference BINARY's stored output needs a GPU: tests/test_gpu_sdfgen.py."""
 import os
 
 import numpy as np

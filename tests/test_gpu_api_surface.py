@@ -74,11 +74,12 @@ def test_training_model_wiring(cuda):
     assert torch.allclose(grid.grid_to_world(ijk.float()), dec_svh.get_voxel_centers(0))
 
 
-def test_headless_example_runs():
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "examples", "recons_simple.py"), "-", "/tmp/recons_simple.obj"],
+def test_headless_example_runs(tmp_path):
+    obj = str(tmp_path / "recons_simple.obj")
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "examples", "recons_simple.py"), "-", obj],
                          capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr[-800:]
-    assert os.path.getsize("/tmp/recons_simple.obj") > 10000
+    assert os.path.getsize(obj) > 10000
 
 
 def test_fields_follow_their_tensors_device():

@@ -1,15 +1,16 @@
 """SURVEY 8(f) row 4 -- the reference's GT-SDF generator ext.sdfgen.sdf_from_points (ext/sdfgen/sdf_from_points.cu,
-ext/common/kdtree_cuda.cu), the ONE piece of this path whose source is in /root/reference:
+ext/common/kdtree_cuda.cu), the ONE piece of this path whose source the reference publishes:
 
   * nksr_b200.sdfgen.sdf_from_points (csrc/sdfgen.cu: voxel-hash kNN + vote in one kernel)
   * oracle/sdfgen.py (numpy + cKDTree restatement, line by line)
-  * oracle/_ref/nksr_sdfgen_ref.so -- the UNMODIFIED reference sources compiled for sm_100a by oracle/Makefile.ref
+  * tests/golden/sdfgen/sdf_from_points_reference.npz -- what the UNMODIFIED reference sources (compiled for sm_100a by
+    oracle/Makefile.ref) return on these inputs, at a fixed seeded sample of the queries
+    (tests/golden/make_sdfgen_golden.py)
 
 are compared pairwise on the GPU with the reference's own argument sets (dataset/av_gt_geometry.py:67-70: nb_points=8,
 stdv=3.0, adaptive_knn=8; models/loss.py:85: 8, 0.02) plus the IMLS variant.  The rule is discontinuous where the nearest
 distance crosses stdv*ref_std, where a vote d_k crosses 0 and where the k-th / (k+1)-th neighbours swap: queries within a
 rounding error of such a point are excluded from the exact comparison (and counted: they must be rare)."""
-import importlib.util
 import os
 
 import numpy as np
@@ -20,21 +21,18 @@ from oracle import sdfgen as OS
 from tests import clouds, scenes
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_SO = os.path.join(ROOT, "oracle", "_ref", "nksr_sdfgen_ref.so")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "sdfgen",
+                      "sdf_from_points_reference.npz")
+SAMPLE = 1500            # queries per case whose reference output is stored
 
 
 def _np(t):
     return t.detach().cpu().numpy()
 
 
-def _reference_module():
-    if not os.path.exists(REF_SO):
-        return None
-    spec = importlib.util.spec_from_file_location("nksr_sdfgen_ref", REF_SO)
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    return mod
+def sample_indices(m):
+    """the fixed, seeded sample of the queries at which the reference output is stored"""
+    return np.sort(np.random.default_rng(11).choice(m, SAMPLE, replace=False))
 
 
 def _case(name):
@@ -54,14 +52,16 @@ def _case(name):
     return xyz.astype(np.float32), nrm.astype(np.float32), q
 
 
+CASES = ["sphere", "cfg4"]
 ARGS = [dict(nb_points=8, stdv=3.0, adaptive_knn=8, imls=False),        # dataset/av_gt_geometry.py:67-70
         dict(nb_points=8, stdv=0.02, adaptive_knn=0, imls=False),       # models/loss.py:85
         dict(nb_points=16, stdv=0.05, adaptive_knn=0, imls=True),
         dict(nb_points=33, stdv=2.0, adaptive_knn=40, imls=False)]
+ARG_IDS = ["gt_geometry", "loss", "imls", "k33"]
 
 
-@pytest.mark.parametrize("case", ["sphere", "cfg4"])
-@pytest.mark.parametrize("args", ARGS, ids=["gt_geometry", "loss", "imls", "k33"])
+@pytest.mark.parametrize("case", CASES)
+@pytest.mark.parametrize("args", ARGS, ids=ARG_IDS)
 def test_sdf_from_points_matches_reference_and_oracle(cuda, case, args):
     import nksr_b200
     xyz, nrm, q = _case(case)
@@ -80,13 +80,14 @@ def test_sdf_from_points_matches_reference_and_oracle(cuda, case, args):
     assert (np.abs(sdf - o_sdf)[clear] <= tol[clear]).all(), np.abs(sdf - o_sdf)[clear].max()
     assert np.abs(grad - o_grad)[clear].max() <= 2e-4
     assert (np.abs(sdf - o_sdf) <= tol).mean() >= 0.99
-    ref = _reference_module()
-    if ref is None:      # kernel and restatement agree (above); the binary that pins both did not travel to this box
-        pytest.skip("oracle/_ref/nksr_sdfgen_ref.so missing: `make -C oracle -f Makefile.ref` (build() does it where "
-                    "/root/reference exists)")
-    r = ref.sdf_from_points(t(q), t(xyz), t(nrm), kw["nb_points"], kw["stdv"], True, kw["imls"], kw["adaptive_knn"])
-    r_sdf, r_grad = _np(r[0]), _np(r[1])
-    # the oracle is pinned by the reference binary, and so is the kernel
+    # the oracle is pinned by the reference binary's output, and so is the kernel
+    g = np.load(GOLDEN)
+    tag = f"{case}_{ARG_IDS[ARGS.index(args)]}"
+    i = sample_indices(q.shape[0])
+    assert np.allclose(q[i], g[f"{case}_q"], rtol=0, atol=1e-5), "the seeded inputs are not the ones the reference " \
+                                                                 "output was stored for"
+    r_sdf, r_grad = g[f"{tag}_sdf"], g[f"{tag}_grad"]
+    o_sdf, sdf, grad, clear, tol = o_sdf[i], sdf[i], grad[i], clear[i], tol[i]
     assert (np.abs(o_sdf - r_sdf)[clear] <= tol[clear]).all(), np.abs(o_sdf - r_sdf)[clear].max()
     assert (np.abs(sdf - r_sdf)[clear] <= tol[clear]).all(), np.abs(sdf - r_sdf)[clear].max()
     assert np.abs(grad - r_grad)[clear].max() <= 2e-4
